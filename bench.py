@@ -79,6 +79,27 @@ def peaks():
     return dict(hbm=6650.0, tf=1590.0, tf_sus=1400.0, src='fallback')
 
 
+DUMP_BYTES = 60 * 10 ** 6          # --dump-outputs: stays under 64 MB with the .npy headers
+
+
+def dump_outputs(path, arrays):
+    """Write name -> tensor as <path>/<name>.npy: float64 and integer outputs as float64, the others as float32.  An
+    output larger than its share of what is left of DUMP_BYTES (smallest outputs first) keeps a fixed sample of its
+    flattened elements: the first indices of torch.randperm under seed 0, in ascending order."""
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_BYTES
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    for i, (name, t) in enumerate(items):
+        t = t.detach().cpu()
+        t = t.double() if t.dtype == torch.float64 or not t.is_floating_point() else t.float()
+        share = left // (len(items) - i) // t.element_size()
+        if t.numel() > share:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:share].sort().values
+            t = t.reshape(-1)[idx]
+        np.save(os.path.join(path, name + '.npy'), t.numpy())
+        left -= t.numel() * t.element_size()
+
+
 def build_models(device):
     import projects.mmdet3d_plugin  # noqa: F401  (registers the plug-in classes)
     from projects.mmdet3d_plugin.registry import load_config, build_hot_path
@@ -214,20 +235,17 @@ def run_reference(args):
     fr = host_frame(args.batch, args.cloud, SEED)
     fr = dict(img_feats=fr['img_feats'].clone(), pts_feats=fr['pts_feats'].clone(), img_metas=fr['img_metas'],
               pts_metas=fr['pts_metas'])
-    t0 = time.perf_counter()
     try:
         with Deadline(170):
-            forward(neck, head, fr)                  # warm-up step (also sizes the bounded sample)
+            forward(neck, head, fr)                  # warm-up step
     except TimeoutError:
         print(json.dumps(dict(impl='reference', unavailable='oracle frame did not finish within 170 s on this host')))
         return
-    t1 = time.perf_counter() - t0
-    budget = 100.0
-    steps = max(1, min(args.steps, int(budget / max(t1, 1e-3))))
+    steps = args.steps
     warm = 1
     t0 = time.perf_counter()
     for _ in range(steps):
-        forward(neck, head, fr)
+        out = forward(neck, head, fr)
     dt = (time.perf_counter() - t0) / steps
     fps = args.batch / dt
     line = dict(metric=METRIC, value=fps, unit='frames/s', n_gpus=args.gpus, steps=steps, warmup=warm,
@@ -236,9 +254,11 @@ def run_reference(args):
                 config=dict(workload=WORKLOAD, global_batch=args.batch, cloud=args.cloud, device='host CPU',
                             note='reference math restated in PyTorch (oracle/), all host threads'),
                 cpu_baseline=dict(value=fps, unit='frames/s', cores=cores, kind='port',
-                                  sample=f'{steps} full frame(s) of the same workload (bounded to ~{budget:.0f} s)'),
+                                  sample=f'{steps} full frame(s) of the same workload'),
                 e2e=dict(value=fps, unit='frames/s', h2d_bytes_per_step=0, d2h_bytes_per_step=0), gpu_launches=0)
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
 
 
 def randomize_deform(model, seed):
@@ -318,7 +338,7 @@ def run_plusplus(args):
     def fwd(d):
         o = enc(d)
         return o if head is None else head(o[1], o[0], d['img_metas'])
-    results = lambda o: (o[0], o[1][0], o[1][1]) if head is None else tuple(o[0][0].values())
+    results = lambda o: dict(img_feats=o[0], pts_feats_0=o[1][0], pts_feats_1=o[1][1]) if head is None else o[0][0]
     W, K = max(args.warmup, 3), args.steps
     for _ in range(3):
         for d in devs:
@@ -349,10 +369,11 @@ def run_plusplus(args):
         barrier()
         launches = ops.LAUNCHES[0] - l0
         ms = max_over_ranks(e0.elapsed_time(e1))
+        dumped = {k: v.cpu() for k, v in results(out).items()} if args.dump_outputs else None
         # end to end: host -> device copies of every input of the step, forward, device -> host of the three outputs
         flat = lambda fr: list(fr['img_levels']) + list(fr['pts_levels'])
         dset = dict(img=[torch.empty_like(t) for t in devs[0]['img']], pts=[torch.empty_like(t) for t in devs[0]['pts']])
-        outs_host = [torch.empty(o.shape, dtype=o.dtype).pin_memory() for o in results(out)]
+        outs_host = [torch.empty(o.shape, dtype=o.dtype).pin_memory() for o in results(out).values()]
         h2d_b = int(np.mean([sum(t.numel() * 4 for t in flat(f)) + sum(v.numel() * v.element_size() for k_, v in
                              f['pts_metas'].items() if k_ != 'pts') + sum(p.numel() * 4 for p in f['pts_metas']['pts'])
                              for f in hosts]))
@@ -365,7 +386,7 @@ def run_plusplus(args):
             o = fwd(dict(img=dset['img'], pts=dset['pts'], img_metas=fh['img_metas'],
                          pts_metas=dict(pillars=nb(pm['pillars']), pillar_coors=nb(pm['pillar_coors']),
                                         pillars_num_points=nb(pm['pillars_num_points']), pts=[nb(p) for p in pm['pts']])))
-            for dst, src in zip(outs_host, results(o)):
+            for dst, src in zip(outs_host, results(o).values()):
                 dst.copy_(src, non_blocking=True)
         for i in range(3):
             e2e_step(i)
@@ -443,6 +464,8 @@ def run_plusplus(args):
                                         d2h_bytes_per_step=int(sum(t.numel() * 4 for t in outs_host)), ms_per_step=ms_e2e / K),
                 gpu_launches=launches, launches_per_step=launches / K, roofline=roof, cpu_baseline=cpu, kernels=kernels[:12])
     print(json.dumps(line), flush=True)
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 
@@ -495,7 +518,7 @@ def run_large(args):
 
     def fwd(d):
         img, pts = neck(d['img'], d['pts'], d['img_metas'], dict(pts=d['cloud']))
-        return (img, pts[0], pts[1]) if head is None else tuple(head(pts, img, d['img_metas'])[0][0].values())
+        return dict(img_feats=img, pts_feats_0=pts[0], pts_feats_1=pts[1]) if head is None else head(pts, img, d['img_metas'])[0][0]
     W, K = max(args.warmup, 3), args.steps
     for _ in range(3):
         for d in devs:
@@ -526,8 +549,9 @@ def run_large(args):
         barrier()
         launches = ops.LAUNCHES[0] - l0
         ms = max_over_ranks(e0.elapsed_time(e1))
+        dumped = {k: v.cpu() for k, v in out.items()} if args.dump_outputs else None
         dset = dict(img=torch.empty_like(devs[0]['img']), pts=torch.empty_like(devs[0]['pts']))
-        outs_host = [torch.empty(o.shape, dtype=o.dtype).pin_memory() for o in out]
+        outs_host = [torch.empty(o.shape, dtype=o.dtype).pin_memory() for o in out.values()]
         h2d_b = int(np.mean([sum(t.numel() * 4 for t in [f['img'], f['pts']] + f['cloud']) for f in hosts]))
 
         def e2e_step(i):
@@ -535,7 +559,7 @@ def run_large(args):
             dset['img'].copy_(fh['img'], non_blocking=True)
             dset['pts'].copy_(fh['pts'], non_blocking=True)
             o = fwd(dict(img=dset['img'], pts=dset['pts'], img_metas=fh['img_metas'], cloud=[nb(p) for p in fh['cloud']]))
-            for dst, src in zip(outs_host, o):
+            for dst, src in zip(outs_host, o.values()):
                 dst.copy_(src, non_blocking=True)
         for i in range(3):
             e2e_step(i)
@@ -594,6 +618,8 @@ def run_large(args):
                                         ms_per_step=ms_e2e / K),
                 gpu_launches=launches, launches_per_step=launches / K, roofline=roof, cpu_baseline=None, kernels=kernels[:12])
     print(json.dumps(line), flush=True)
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 
@@ -618,7 +644,12 @@ def main():
     ap.add_argument('--inflight', type=int, default=5, help='independent frames in flight per GPU (CUDA streams)')
     ap.add_argument('--frames', type=int, default=9, help='distinct synthetic frames (different point / pillar counts) cycled '
                     'through the timed regions, each in its own device buffers')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the outputs of the last timed step as DIR/<name>.npy (at most 64 MB '
+                         'in all; larger outputs keep a fixed, seeded sample of their elements)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         return run_reference(args)
     if args.workload == 'plusplus':
@@ -692,6 +723,7 @@ def main():
         barrier()
         launches = ops.LAUNCHES[0] - l0
         ms = max_over_ranks(e0.elapsed_time(e1))
+        dumped = {k: v.cpu() for k, v in out.items()} if args.dump_outputs else None     # before region 2 reuses the buffers
         # ---- timed region 2: end to end through the plug-in API, host buffers ------------------------------
         # NSETS device input sets; the host->device copy of a later step runs on a copy stream while earlier steps
         # compute on the pipeline's streams; every step's result goes back to pinned host memory on its own stream.
@@ -930,6 +962,8 @@ def main():
                 roofline=roof, modules=modules, cpu_baseline=cpu,
                 kernels=kernels[:12])
     print(json.dumps(line), flush=True)
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 

@@ -8,10 +8,18 @@ import torch
 import torch.nn.functional as F
 
 from conftest import rel_err
+from tools.ref_goldens import REF_CONFIGS, ref_config
 
-REF_CFG = '/root/reference/projects/configs/nuscenes/Fusion_0075_refactor.py'
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OUR_CFG = os.path.join(ROOT, 'projects', 'configs', 'nuscenes', 'di_b200_base_hotpath.py')
+
+
+def load_cfg(src):
+    """A config file of this repository, or a reference config by name (its plug-in part, tests/golden/ref_configs.pt)."""
+    from projects.mmdet3d_plugin.registry import load_config
+    if src in REF_CONFIGS:
+        return ref_config(src)
+    return load_config(src if os.path.isabs(src) else os.path.join(ROOT, src))
 
 
 def test_conv_bn_and_fuse_pair_folding():
@@ -206,15 +214,13 @@ def test_camera_rows_project_like_the_oracle():
     assert float((u2 - uv[..., 0])[vis].abs().max()) < 2e-2
 
 
-@pytest.mark.parametrize('cfg_path', [OUR_CFG, REF_CFG])
-def test_plugin_builds_from_config_with_reference_state_dict_schema(cfg_path):
-    if not os.path.exists(cfg_path):
-        pytest.skip('reference tree not mounted here')
+@pytest.mark.parametrize('cfg_src', [OUR_CFG, 'Fusion_0075_refactor'])
+def test_plugin_builds_from_config_with_reference_state_dict_schema(cfg_src):
     import projects.mmdet3d_plugin  # noqa: F401
-    from projects.mmdet3d_plugin.registry import load_config, build_hot_path, NECKS, HEADS, BBOX_CODERS
+    from projects.mmdet3d_plugin.registry import build_hot_path, NECKS, HEADS, BBOX_CODERS
     import oracle.mmri as om
     import oracle.mmpi as omp
-    cfg = load_config(cfg_path)
+    cfg = load_cfg(cfg_src)
     assert cfg['plugin'] is True and cfg['plugin_dir'] == 'projects/mmdet3d_plugin/'
     neck, head = build_hot_path(cfg)
     assert type(neck).__name__ == 'DeepInteractionEncoder' and type(head).__name__ == 'DeepInteractionDecoder'
@@ -237,16 +243,14 @@ def test_plugin_builds_from_config_with_reference_state_dict_schema(cfg_path):
 
 
 def test_plusplus_config_builds_its_neck_with_the_reference_schema():
-    """The reference's UNCHANGED Fusion_0075_plusplus.py builds `imgpts_neck` (FusionTransformerv4 + DeepInteractionLayer
-    + MMRI_P2I / MMRI_I2P / MMRI_I2P_Polar) through the plug-in registries; state_dict keys and shapes equal the
-    oracle's, whose state_dict tools/make_goldens_pp.py loads strictly into the reference classes."""
-    ref_cfg = '/root/reference/projects/configs/nuscenes/Fusion_0075_plusplus.py'
-    if not os.path.exists(ref_cfg):
-        pytest.skip('reference tree not mounted here')
+    """The reference's unchanged Fusion_0075_plusplus.py (as stored in tests/golden/ref_configs.pt) builds `imgpts_neck`
+    (FusionTransformerv4 + DeepInteractionLayer + MMRI_P2I / MMRI_I2P / MMRI_I2P_Polar) through the plug-in registries;
+    state_dict keys and shapes equal the oracle's, whose state_dict tools/make_goldens_pp.py loads strictly into the
+    reference classes."""
     import projects.mmdet3d_plugin  # noqa: F401
-    from projects.mmdet3d_plugin.registry import load_config, build_neck, NECKS, TRANSFORMER_LAYER, ATTENTION
+    from projects.mmdet3d_plugin.registry import build_neck, NECKS, TRANSFORMER_LAYER, ATTENTION
     import oracle.mmri_pp as opp
-    cfg = load_config(ref_cfg)
+    cfg = load_cfg('Fusion_0075_plusplus')
     neck = build_neck(cfg)
     assert type(neck).__name__ == 'FusionTransformerv4'
     o = opp.FusionTransformerv4(**{k: v for k, v in cfg['model']['imgpts_neck'].items() if k != 'type'})
@@ -261,20 +265,15 @@ def test_plusplus_config_builds_its_neck_with_the_reference_schema():
             assert reg.get(n) is not None, n
 
 
-@pytest.mark.parametrize('cfg_path', ['/root/reference/projects/configs/nuscenes/Fusion_0075_plusplus.py',
-                                      'projects/configs/nuscenes/di_b200_plusplus_hotpath.py'])
-def test_plusplus_config_builds_its_head_with_the_reference_schema(cfg_path):
+@pytest.mark.parametrize('cfg_src', ['Fusion_0075_plusplus', 'projects/configs/nuscenes/di_b200_plusplus_hotpath.py'])
+def test_plusplus_config_builds_its_head_with_the_reference_schema(cfg_src):
     """`pts_bbox_head` of the ++ config (DeepInteractionPlusPlusDecoder: V2 RCNN blocks with ffn / self_ffn / self_norm /
     scale / self_scale, prediction heads on C channels) builds through HEADS; state_dict keys and shapes equal the
     oracle's, whose state_dict tools/make_goldens.py (G7) loads strictly into the reference class."""
-    if not os.path.isabs(cfg_path):
-        cfg_path = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), cfg_path)
-    if not os.path.exists(cfg_path):
-        pytest.skip('reference tree not mounted here')
     import projects.mmdet3d_plugin  # noqa: F401
-    from projects.mmdet3d_plugin.registry import load_config, build_hot_path, HEADS
+    from projects.mmdet3d_plugin.registry import build_hot_path, HEADS
     import oracle.mmpi_pp as opp
-    cfg = load_config(cfg_path)
+    cfg = load_cfg(cfg_src)
     neck, head = build_hot_path(cfg)
     assert type(neck).__name__ == 'FusionTransformerv4' and type(head).__name__ == 'DeepInteractionPlusPlusDecoder'
     assert HEADS.get('DeepInteractionPlusPlusDecoder') is not None
@@ -302,11 +301,9 @@ def test_assigner_and_cost_names_are_registered():
                                   cls_cost=dict(type='FocalLossCost', gamma=2, alpha=0.25, weight=0.15),
                                   reg_cost=dict(type='BBoxBEVL1Cost', weight=0.25), iou_cost=dict(type='IoU3DCost', weight=0.25)))
     assert (a.cls_cost.weight, a.reg_cost.weight, a.reg_cost.kind, a.iou_cost.weight) == (0.15, 0.25, 0, 0.25)
-    ref_cfg = '/root/reference/projects/configs/nuscenes/Fusion_0075_refactor.py'
-    if os.path.exists(ref_cfg):
-        from projects.mmdet3d_plugin.registry import load_config, build_hot_path
-        _, head = build_hot_path(load_config(ref_cfg))
-        assert type(head.bbox_assigner).__name__ == 'HungarianAssigner3D' and head.train_cfg['pos_weight'] == -1
+    from projects.mmdet3d_plugin.registry import build_hot_path
+    _, head = build_hot_path(load_cfg('Fusion_0075_refactor'))
+    assert type(head.bbox_assigner).__name__ == 'HungarianAssigner3D' and head.train_cfg['pos_weight'] == -1
 
 
 def test_product_modules_refuse_cpu_and_training():
